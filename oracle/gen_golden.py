@@ -210,7 +210,7 @@ def gen_generator_extra():
     np.savez_compressed(os.path.join(OUT, 'generator_extra.npz'), **out)
 
 
-GRAD_STRIDE, DISC_GRAD_STRIDE = 7, 211     # gradients are stored subsampled plus their exact L2 norm
+GRAD_STRIDE, DISC_GRAD_STRIDE = 7, 633     # gradients are stored subsampled plus their exact L2 norm (keeps each fixture under 1 MB)
 
 
 def grad_stride(numel, stride):
@@ -529,6 +529,39 @@ def gen_svb_vae():
     print('svb_vae.npz', out['a2p_mel'].shape, float(np.abs(out['a2p_mel']).max()), len(keys), 'state keys')
 
 
+HPARAMS_CASES = [('egs/egs_bases/tts/vocoder/hifigan.yaml', 'hop_size=128'),
+                 ('egs/datasets/audio/PopBuTFy/vae_global_mle_eng.yaml', 'hop_size=128')]
+
+
+def gen_hparams():
+    """The reference's set_hparams (utils/hparams.py) on base_config chains of its egs/ tree: every YAML file it opened, stored
+    parsed (the resolver reads them with yaml.safe_load), and the dict it returned for each (config, --hparams) case."""
+    import builtins
+    import importlib.util
+    import json
+    import yaml
+    spec = importlib.util.spec_from_file_location('ref_hparams', os.path.join(R.REF_ROOT, 'utils', 'hparams.py'))
+    ref = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(ref)
+    opened = []
+    ref.open = lambda fn, *a, **k: (opened.append(fn), builtins.open(fn, *a, **k))[1]
+    cwd = os.getcwd()
+    os.chdir(R.REF_ROOT)
+    try:
+        cases = [{'config': cfg, 'hparams_str': hs,
+                  'resolved': ref.set_hparams(cfg, hparams_str=hs, print_hparams=False, global_hparams=False)}
+                 for cfg, hs in HPARAMS_CASES]
+        files = {fn: yaml.safe_load(open(fn)) for fn in sorted(set(opened))}
+    finally:
+        os.chdir(cwd)
+    out = {'files': files, 'cases': cases}
+    assert json.loads(json.dumps(out)) == out, 'a resolved value does not survive JSON'
+    with open(os.path.join(OUT, 'hparams.json'), 'w') as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write('\n')
+    print('hparams.json', len(files), 'YAML files,', [len(c['resolved']) for c in cases], 'resolved keys')
+
+
 def main():
     if not R.available():
         sys.exit('gen_golden needs /root/reference (build container only)')
@@ -536,7 +569,7 @@ def main():
     torch.set_num_threads(max(1, os.cpu_count() or 1))
     warnings.simplefilter('ignore')
     which = sys.argv[1:] or ['frontend', 'generator', 'losses', 'discriminators', 'discriminators_cond', 'generator_extra',
-                             'generator_grads', 'losses_extra', 'discriminators_train', 'wn', 'fvae_decoder', 'fvae_encoder', 'global_fvae', 'vc_asr', 'svb_vae']
+                             'generator_grads', 'losses_extra', 'discriminators_train', 'wn', 'fvae_decoder', 'fvae_encoder', 'global_fvae', 'vc_asr', 'svb_vae', 'hparams']
     for w in which:
         globals()[f'gen_{w}']()
 

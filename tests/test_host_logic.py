@@ -41,17 +41,20 @@ def test_hparams_chain_override_and_cli(tmp_path, monkeypatch):
     assert hp2['x'] == 9 and hp2['work_dir'] == 'checkpoints/e1'
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/egs'), reason='reference mount only in the build container')
-def test_hparams_resolves_reference_yaml_like_the_reference(monkeypatch):
-    import importlib.util
-    monkeypatch.chdir('/root/reference')
-    spec = importlib.util.spec_from_file_location('ref_hparams', '/root/reference/utils/hparams.py')
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    for cfg in ('egs/egs_bases/tts/vocoder/hifigan.yaml', 'egs/datasets/audio/PopBuTFy/vae_global_mle_eng.yaml'):
-        a = HP.set_hparams(cfg, hparams_str='hop_size=128', print_hparams=False, global_hparams=False)
-        b = ref.set_hparams(cfg, hparams_str='hop_size=128', print_hparams=False, global_hparams=False)
-        assert a == b
+def test_hparams_resolves_reference_yaml_like_the_reference(golden_dir, tmp_path, monkeypatch):
+    """base_config chains of the reference's egs/ tree resolve to the dict the reference's set_hparams returned
+    (tests/golden/hparams.json, written by oracle/gen_golden.py gen_hparams: the YAML files parsed, and the resolved dicts)."""
+    import json
+    import yaml
+    gold = json.load(open(os.path.join(golden_dir, 'hparams.json')))
+    for rel, content in gold['files'].items():
+        (tmp_path / rel).parent.mkdir(parents=True, exist_ok=True)
+        (tmp_path / rel).write_text(yaml.safe_dump(content, sort_keys=False))
+    monkeypatch.chdir(tmp_path)
+    assert len(gold['cases']) == 2
+    for case in gold['cases']:
+        a = HP.set_hparams(case['config'], hparams_str=case['hparams_str'], print_hparams=False, global_hparams=False)
+        assert a == case['resolved']
 
 
 def test_generator_state_dict_layout_is_the_checkpoint_contract():
