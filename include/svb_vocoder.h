@@ -124,6 +124,24 @@ int svb_gen_spec2wav_host_i16(svb_gen_t *g, const float *mel_host, const float *
 /* the conversion alone on device buffers: wav_dev fp32 [B, n] -> out_dev int16 [B, n] (stream-ordered). */
 int svb_wav_to_int16(const float *wav_dev, int32_t B, int64_t n, int32_t norm, int16_t *out_dev, void *stream);
 
+/* HifiGanGenerator.forward over clips of different lengths (padded device layout, like MleSVBVAE's output):
+ *   mel_dev [B, n_mel, T_max], f0_dev [B, T_max] or NULL, lengths_host int32 [B] in [1, T_max],
+ *   rand_ini_dev [B, 9] / noise_dev [B, T_max*hop, 9] or both NULL (Philox keyed by (t, b, harmonic) as in svb_gen_forward),
+ *   wav_dev [B, T_max*hop]: clip b's first lengths[b]*hop samples, zeros after.  Values past a clip's length in
+ *   mel / f0 / noise are never read.  Clip b's samples are bit-identical to a forward of that clip alone (same
+ *   injected noise); tiles wholly past a clip's end are not computed.  Inference only: a handle in training mode
+ *   returns SVB_ERR_INVALID.  Stream-ordered, no host synchronisation. */
+int svb_gen_forward_ragged(svb_gen_t *g, const float *mel_dev, const float *f0_dev, const int32_t *lengths_host,
+                           const float *rand_ini_dev, const float *noise_dev, uint64_t seed, int32_t B, int32_t T_max,
+                           float *wav_dev, void *stream);
+/* spec2wav over a ragged batch from HOST memory: mel_host [sum T_b, n_mel] and f0_host [sum T_b] (or NULL) clip after clip,
+ * wav_host [sum T_b * hop] clip after clip (svb_wav2spec_batch_host's convention).  Synchronises `stream`. */
+int svb_gen_spec2wav_ragged_host(svb_gen_t *g, const float *mel_host, const float *f0_host, const int32_t *lengths_host,
+                                 int32_t B, uint64_t seed, float *wav_host, void *stream);
+/* the same with save_wav's int16 conversion on the device; `norm` takes each clip's peak over its own samples. */
+int svb_gen_spec2wav_ragged_host_i16(svb_gen_t *g, const float *mel_host, const float *f0_host, const int32_t *lengths_host,
+                                     int32_t B, uint64_t seed, int32_t norm, int16_t *wav_host, void *stream);
+
 /* Intermediate tap for layer-level parity tests: copies a named activation of the LAST forward
  * ("har_source" [B,T*hop]; "conv_pre", "ups{i}", "stage{i}" as [B,C,T_i]) to out_dev. */
 int svb_gen_get_tap(svb_gen_t *g, const char *name, float *out_dev, int64_t capacity_floats,
@@ -373,6 +391,11 @@ int svb_relpos_attention_nct(const float *q_dev, const float *k_dev, const float
 int64_t svb_tc_schedule_probe(int32_t n_layers, const int32_t *KS, const int32_t *has_res, const int32_t *accumulate, int32_t Cin, int32_t B,
                               int32_t Tq, int32_t MT, int32_t col_blocks, int32_t chain_ordered, int32_t grid, int32_t *items_out,
                               int64_t items_capacity, int32_t *off_out, double *balance_out);
+/* svb_tc_schedule_probe for a ragged batch: clip b has rows_per_clip[b] >= 1 rows (and only its own tiles). */
+int64_t svb_tc_schedule_probe_ragged(int32_t n_layers, const int32_t *KS, const int32_t *has_res, const int32_t *accumulate,
+                                     int32_t Cin, int32_t B, const int32_t *rows_per_clip, int32_t MT, int32_t col_blocks,
+                                     int32_t chain_ordered, int32_t grid, int32_t *items_out, int64_t items_capacity,
+                                     int32_t *off_out, double *balance_out);
 
 #ifdef __cplusplus
 }

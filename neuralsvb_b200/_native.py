@@ -158,6 +158,11 @@ _PROTOS = {
     'svb_fvae_decoder_create': (ctypes.c_int, [_I32, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _I32, ctypes.POINTER(_P)]),
     'svb_fvae_decoder_forward': (ctypes.c_int, [_P, _P, _P, _P, _I32, _I32, _P, _P]),
     'svb_tc_schedule_probe': (_I64, [_I32, _P, _P, _P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _I64, _P, ctypes.POINTER(ctypes.c_double)]),
+    'svb_tc_schedule_probe_ragged': (_I64, [_I32, _P, _P, _P, _I32, _I32, _P, _I32, _I32, _I32, _I32, _P, _I64, _P,
+                                            ctypes.POINTER(ctypes.c_double)]),
+    'svb_gen_forward_ragged': (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _U64, _I32, _I32, _P, _P]),
+    'svb_gen_spec2wav_ragged_host': (ctypes.c_int, [_P, _P, _P, _P, _I32, _U64, _P, _P]),
+    'svb_gen_spec2wav_ragged_host_i16': (ctypes.c_int, [_P, _P, _P, _P, _I32, _U64, _I32, _P, _P]),
     'svb_layer_norm_nct': (ctypes.c_int, [_P, _P, _P, _I32, _I32, _I32, ctypes.c_float, _P, _P]),
     'svb_relpos_attention_nct': (ctypes.c_int, [_P, _P, _P, _P, _P, _P, _P, _I32, _I32, _I32, _I32, _P, _P]),
 }

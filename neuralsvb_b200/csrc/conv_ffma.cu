@@ -6,6 +6,8 @@
 // Input channels are consumed 16 at a time through shared memory; the leaky-relu pre-activation
 // of the ResBlocks (hifigan.py:55,57) is applied while staging, bias / residual / 1/num_kernels
 // scaling / ResBlock-sum accumulation are fused in the epilogue.
+#include <algorithm>
+
 #include "conv_ffma.cuh"
 
 namespace svb {
@@ -29,6 +31,8 @@ __global__ void __launch_bounds__(256) conv1d_c4_ffma_kernel(ConvArgs a) {
     const int co0 = co_tile0 + warp * CPT;                     // first GEMM column of this warp
     const bool active = co0 < a.CoutP;
     const int cin_q = a.Cin >> 2;
+    const int Tq = valid_rows(a, b);
+    if (t0 >= Tq) return;                                      // tile wholly past this clip's end (ragged batch)
 
     float acc[kRowsPerThread][CPT];
 #pragma unroll
@@ -104,7 +108,7 @@ __global__ void __launch_bounds__(256) conv1d_c4_ffma_kernel(ConvArgs a) {
 #pragma unroll
         for (int r = 0; r < kRowsPerThread; ++r) {
             const int q = t0 + lane + 32 * r;
-            if (q >= a.Tq) continue;
+            if (q >= Tq) continue;
             const size_t row = act_q4(b, a.Cout, a.out_Tp, co >> 2, kPad + (a.ups_u > 0 ? q * a.ups_u + phi : q));
             float4 v = make_float4(acc[r][4 * c4 + 0] + bv.x, acc[r][4 * c4 + 1] + bv.y,
                                    acc[r][4 * c4 + 2] + bv.z, acc[r][4 * c4 + 3] + bv.w);
@@ -164,12 +168,17 @@ int launch_conv_ffma(const ConvArgs &a, cudaStream_t st) {
 }
 
 // ------------------------------------------------------------------------------ layout changes
-__global__ void nct_to_c4t_kernel(const float *__restrict__ nct, float4 *__restrict__ c4t, int C, int T, int Tp) {
+__global__ void nct_to_c4t_kernel(const float *__restrict__ nct, float4 *__restrict__ c4t, int C, int T, int Tp,
+                                  const int *__restrict__ len) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int cq = blockIdx.y, b = blockIdx.z;
     if (t >= T) return;
-    const float *p = nct + ((size_t)b * C + cq * 4) * T + t;
-    c4t[act_q4(b, C, Tp, cq, kPad + t)] = make_float4(p[0], p[T], p[2 * (size_t)T], p[3 * (size_t)T]);
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!len || t < len[b]) {
+        const float *p = nct + ((size_t)b * C + cq * 4) * T + t;
+        v = make_float4(p[0], p[T], p[2 * (size_t)T], p[3 * (size_t)T]);
+    }
+    c4t[act_q4(b, C, Tp, cq, kPad + t)] = v;
 }
 
 __global__ void c4t_to_nct_kernel(const float4 *__restrict__ c4t, float *__restrict__ nct, int C, int T, int Tp) {
@@ -181,17 +190,19 @@ __global__ void c4t_to_nct_kernel(const float4 *__restrict__ c4t, float *__restr
     p[0] = v.x, p[T] = v.y, p[2 * (size_t)T] = v.z, p[3 * (size_t)T] = v.w;
 }
 
-__global__ void btc_to_c4t_kernel(const float4 *__restrict__ btc, float4 *__restrict__ c4t, int C, int T, int Tp) {
+__global__ void btc_to_c4t_kernel(const float4 *__restrict__ btc, float4 *__restrict__ c4t, int C, int T, int Tp, Ragged rg) {
     // one thread per (t, quad): reads 16 B of the frame-major row, writes one C4T row
     const int cq = blockIdx.x * blockDim.x + threadIdx.x;
     const int t = blockIdx.y, b = blockIdx.z;
     if (cq >= (C >> 2)) return;
-    c4t[act_q4(b, C, Tp, cq, kPad + t)] = btc[((size_t)b * T + t) * (C >> 2) + cq];
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!rg.len || t < rg.len[b]) v = btc[((rg.off ? (size_t)rg.off[b] : (size_t)b * T) + t) * (C >> 2) + cq];
+    c4t[act_q4(b, C, Tp, cq, kPad + t)] = v;
 }
 
-int launch_nct_to_c4t(const float *nct, float *c4t, int B, int C, int T, int Tp, cudaStream_t st) {
+int launch_nct_to_c4t(const float *nct, float *c4t, int B, int C, int T, int Tp, cudaStream_t st, Ragged rg) {
     dim3 grid((T + 127) / 128, C / 4, B);
-    nct_to_c4t_kernel<<<grid, 128, 0, st>>>(nct, reinterpret_cast<float4 *>(c4t), C, T, Tp);
+    nct_to_c4t_kernel<<<grid, 128, 0, st>>>(nct, reinterpret_cast<float4 *>(c4t), C, T, Tp, rg.len);
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }
@@ -201,10 +212,10 @@ int launch_c4t_to_nct(const float *c4t, float *nct, int B, int C, int T, int Tp,
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }
-int launch_btc_to_c4t(const float *btc, float *c4t, int B, int C, int T, int Tp, cudaStream_t st) {
+int launch_btc_to_c4t(const float *btc, float *c4t, int B, int C, int T, int Tp, cudaStream_t st, Ragged rg) {
     dim3 grid((C / 4 + 31) / 32, T, B);
     btc_to_c4t_kernel<<<grid, 32, 0, st>>>(reinterpret_cast<const float4 *>(btc), reinterpret_cast<float4 *>(c4t), C,
-                                           T, Tp);
+                                           T, Tp, rg);
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }
@@ -214,10 +225,12 @@ int launch_btc_to_c4t(const float *btc, float *c4t, int B, int C, int T, int Tp,
 // a warp touches 4 whole 128-byte rows; har[] is a broadcast within a row; nw is packed [K][C].
 __global__ void noise_conv_add_kernel(float4 *__restrict__ x, int C, int T, int Tp, const float *__restrict__ har,
                                       int Thar, const float *__restrict__ nw, const float *__restrict__ nb, int K,
-                                      int stride, int pad) {
+                                      int stride, int pad, const int *__restrict__ len, int x_mul, int har_mul) {
     const int cq_n = c4t_groups(C) * 8;                       // quads per row incl. zero padding channels
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int b = blockIdx.y;
+    const int Hb = len ? len[b] * har_mul : Thar;             // har samples of this clip
+    if (len) T = len[b] * x_mul;
     if (idx >= (long long)T * cq_n) return;
     const int n = (int)(idx / cq_n), cq = (int)(idx - (long long)n * cq_n);
     if (cq * 4 >= C) return;
@@ -226,7 +239,7 @@ __global__ void noise_conv_add_kernel(float4 *__restrict__ x, int C, int T, int 
     const int base = n * stride - pad;
     for (int j = 0; j < K; ++j) {
         const int i = base + j;
-        if (i < 0 || i >= Thar) continue;
+        if (i < 0 || i >= Hb) continue;
         const float hv = __ldg(h + i);
         const float4 w = __ldg(reinterpret_cast<const float4 *>(nw + (size_t)j * C) + cq);
         acc.x = fmaf(w.x, hv, acc.x), acc.y = fmaf(w.y, hv, acc.y), acc.z = fmaf(w.z, hv, acc.z), acc.w = fmaf(w.w, hv, acc.w);
@@ -238,10 +251,11 @@ __global__ void noise_conv_add_kernel(float4 *__restrict__ x, int C, int T, int 
 }
 
 int launch_noise_conv_add(float *x, int B, int C, int T, int Tp, const float *har, int Thar, const float *nw,
-                          const float *nb, int K, int stride, int pad, cudaStream_t st) {
+                          const float *nb, int K, int stride, int pad, cudaStream_t st, Ragged rg, int x_mul, int har_mul) {
     const long long total = (long long)T * c4t_groups(C) * 8;
     dim3 grid((unsigned)((total + 255) / 256), B);
-    noise_conv_add_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<float4 *>(x), C, T, Tp, har, Thar, nw, nb, K, stride, pad);
+    noise_conv_add_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<float4 *>(x), C, T, Tp, har, Thar, nw, nb, K, stride, pad, rg.len,
+                                                x_mul, har_mul);
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }
@@ -249,12 +263,17 @@ int launch_noise_conv_add(float *x, int B, int C, int T, int Tp, const float *ha
 // ------------------------------------------------------------------------------ conv_post + tanh
 __global__ void __launch_bounds__(256) conv_post_tanh_kernel(const float4 *__restrict__ x, int C, int T, int Tp,
                                                              const float4 *__restrict__ wq, const float *__restrict__ bias, int K,
-                                                             float slope, float *__restrict__ wav) {
+                                                             float slope, float *__restrict__ wav, Ragged rg, int mul) {
     extern __shared__ float4 sm4[];
     const int cq_n = C >> 2, halo = (K - 1) / 2, rows = 256 + 2 * halo;
     float4 *xs = sm4;               // [cq_n][rows]
     float4 *ws = sm4 + cq_n * rows; // [cq_n][K]
     const int b = blockIdx.y, t0 = blockIdx.x * 256, tid = threadIdx.x;
+    // ragged batch: clip b has Tv samples; the padded output gets zeros up to T, the packed one holds the clip alone
+    const int Tv = rg.len ? rg.len[b] * mul : T;
+    float *wb = rg.off ? wav + (size_t)rg.off[b] * mul : wav + (size_t)b * T;
+    if (!rg.off && t0 + tid >= Tv && t0 + tid < T) wb[t0 + tid] = 0.f;
+    if (t0 >= Tv) return;                                   // tile wholly past the clip's end
     for (int idx = tid; idx < cq_n * rows; idx += 256) {
         const int r = idx / cq_n, cq = idx - r * cq_n;      // quads of a row are contiguous in G32T
         xs[cq * rows + r] = lrelu4(__ldg(x + act_q4(b, C, Tp, cq, kPad + t0 - halo + r)), slope);
@@ -262,7 +281,7 @@ __global__ void __launch_bounds__(256) conv_post_tanh_kernel(const float4 *__res
     for (int idx = tid; idx < cq_n * K; idx += 256) ws[idx] = wq[idx];
     __syncthreads();
     const int t = t0 + tid;
-    if (t >= T) return;
+    if (t >= Tv) return;
     float acc = __ldg(bias);
     for (int cq = 0; cq < cq_n; ++cq)
         for (int k = 0; k < K; ++k) {
@@ -270,11 +289,11 @@ __global__ void __launch_bounds__(256) conv_post_tanh_kernel(const float4 *__res
             acc = fmaf(xv.x, wv.x, acc), acc = fmaf(xv.y, wv.y, acc), acc = fmaf(xv.z, wv.z, acc),
             acc = fmaf(xv.w, wv.w, acc);
         }
-    wav[(size_t)b * T + t] = tanhf(acc);
+    wb[t] = tanhf(acc);
 }
 
 int launch_conv_post_tanh(const float *x, int B, int C, int T, int Tp, const float *wq, const float *bias, int K, float slope,
-                          float *wav, cudaStream_t st) {
+                          float *wav, cudaStream_t st, Ragged rg, int mul) {
     const int rows = 256 + (K - 1);
     const size_t smem = (size_t)(C / 4) * (rows + K) * 16;
     SVB_CHECK(smem <= 200 * 1024, SVB_ERR_INVALID, "conv_post: %d channels do not fit shared memory", C);
@@ -285,7 +304,37 @@ int launch_conv_post_tanh(const float *x, int B, int C, int T, int Tp, const flo
     }
     dim3 grid((T + 255) / 256, B);
     conv_post_tanh_kernel<<<grid, 256, smem, st>>>(reinterpret_cast<const float4 *>(x), C, T, Tp,
-                                                   reinterpret_cast<const float4 *>(wq), bias, K, slope, wav);
+                                                   reinterpret_cast<const float4 *>(wq), bias, K, slope, wav, rg, mul);
+    SVB_CUDA(cudaGetLastError());
+    return SVB_OK;
+}
+
+// ------------------------------------------------------------------------------ stale rows of a ragged batch
+struct ZeroSegs {
+    ZeroSeg s[kMaxZeroSegs];
+};
+// grid (row blocks, segment, clip): rows [len[b] * mul, hw[b] * mul) of every channel group of segment y, clip z
+__global__ void zero_tails_kernel(ZeroSegs segs, const int *__restrict__ len, const int *__restrict__ hw) {
+    const ZeroSeg sg = segs.s[blockIdx.y];
+    const int b = blockIdx.z;
+    const int r0 = len[b] * sg.mul, r1 = min(hw[b] * sg.mul, sg.Tp - 2 * kPad);
+    if (r0 >= r1) return;
+    const long long n = (long long)(r1 - r0) * 8 * sg.groups;             // float4s
+    float4 *base = reinterpret_cast<float4 *>(sg.p);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const int q = (int)(i & 7);
+        const long long rg = i >> 3;
+        const int grp = (int)(rg / (r1 - r0)), r = r0 + (int)(rg - (long long)grp * (r1 - r0));
+        base[(((size_t)b * sg.groups + grp) * sg.Tp + kPad + r) * 8 + q] = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+}
+
+int launch_zero_tails(const ZeroSeg *segs, int n, int B, const int *len, const int *hw, int max_rows, cudaStream_t st) {
+    SVB_CHECK(n >= 1 && n <= kMaxZeroSegs, SVB_ERR_INVALID, "zero_tails: %d buffers (limit %d)", n, kMaxZeroSegs);
+    ZeroSegs s;
+    for (int i = 0; i < n; ++i) s.s[i] = segs[i];
+    const dim3 grid((unsigned)std::max(1, std::min((max_rows * 8 + 255) / 256, 64)), (unsigned)n, (unsigned)B);
+    zero_tails_kernel<<<grid, 256, 0, st>>>(s, len, hw);
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }

@@ -107,13 +107,14 @@ __device__ __forceinline__ void mbar_wait_warp(uint64_t *bar, uint32_t parity, l
 }
 constexpr int kTcStatSlots = 16;
 
-// a work item, as staged in shared memory: x = layer | column block << 8 | tiles << 24, y = clip, z = first row
+// a work item, as staged in shared memory: x = layer | column block << 8 | tiles << 24, y = clip, z = first row,
+// w = valid rows of the clip (rows at or past it are not stored; a ragged batch has its own count per clip)
 struct TcItem {
-    int layer, nblk, mt, b, t0;
+    int layer, nblk, mt, b, t0, rows;
 };
 __device__ __forceinline__ TcItem item_decode(const int4 v) {
     TcItem it;
-    it.layer = v.x & 0xff, it.nblk = (v.x >> 8) & 0xffff, it.mt = v.x >> 24, it.b = v.y, it.t0 = v.z;
+    it.layer = v.x & 0xff, it.nblk = (v.x >> 8) & 0xffff, it.mt = v.x >> 24, it.b = v.y, it.t0 = v.z, it.rows = v.w;
     return it;
 }
 
@@ -121,7 +122,9 @@ __device__ __forceinline__ TcItem item_decode(const int4 v) {
 // column block of one layer).  Every stage is decoupled by mbarriers, so the TMA producer runs ahead into
 // the next item, the transform warps prepare operands while the tensor core works on the previous chunk,
 // and the epilogue drains accumulator set (n & 1) from TMEM while the MMAs of item n + 1 fill the other set.
-template <int MODE, bool ST = false>
+// RG: ragged batch (a.rows != nullptr), the epilogue bounds rows by the item's clip; a separate instantiation keeps the
+// uniform kernel's epilogue on the constant a.Tq (one register fewer under the 96-register cap)
+template <int MODE, bool ST = false, bool RG = false>
 __global__ void __launch_bounds__(kTcThreadsP, 1) conv1d_c4_tc_kernel(const __grid_constant__ TcArgs p) {
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr bool BF = MODE == SVB_PREC_BF16X3;
@@ -163,12 +166,23 @@ __global__ void __launch_bounds__(kTcThreadsP, 1) conv1d_c4_tc_kernel(const __gr
             const int i0 = __ldg(p.work_off + blockIdx.x), n = __ldg(p.work_off + blockIdx.x + 1) - i0;
             for (int i = threadIdx.x; i < n; i += kTcThreadsP) it_w[i] = __ldg(p.work + i0 + i);
             if (threadIdx.x == 0) *n_items_s = n;
+        } else if (RG) {                                             // implicit, ragged: only the groups inside each clip
+            if (threadIdx.x == 0) {
+                int n = 0;
+                for (int g = blockIdx.x; g < p.total_groups; g += gridDim.x) {
+                    const int tg = g % p.groups_per_b, r = g / p.groups_per_b, b = r % a.B;
+                    const int rows = a.rows[b] * a.rows_mul, tiles = (rows + kTcM - 1) / kTcM;
+                    if (tg * p.MT >= tiles) continue;
+                    it_w[n++] = make_int4(((r / a.B) << 8) | (min(p.MT, tiles - tg * p.MT) << 24), b, tg * (kTcM * p.MT), rows);
+                }
+                *n_items_s = n;
+            }
         } else {                                                     // implicit: groups blockIdx.x, + gridDim.x, ... of layer 0
             const int n = ((int)blockIdx.x < p.total_groups) ? (p.total_groups - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
             for (int i = threadIdx.x; i < n; i += kTcThreadsP) {
                 const int g = blockIdx.x + i * gridDim.x;
                 const int tg = g % p.groups_per_b, r = g / p.groups_per_b;
-                it_w[i] = make_int4(((r / a.B) << 8) | (p.MT << 24), r % a.B, tg * (kTcM * p.MT), 0);
+                it_w[i] = make_int4(((r / a.B) << 8) | (p.MT << 24), r % a.B, tg * (kTcM * p.MT), a.Tq);
             }
             if (threadIdx.x == 0) *n_items_s = n;
         }
@@ -465,7 +479,7 @@ __global__ void __launch_bounds__(kTcThreadsP, 1) conv1d_c4_tc_kernel(const __gr
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 const int rr = 4 * i + wr;
-                rres[i] = (q_base + rr < a.Tq) ? __ldg(res4 + base + (size_t)rr * rstep + wc) : make_float4(0.f, 0.f, 0.f, 0.f);
+                rres[i] = (q_base + rr < (RG ? it.rows : a.Tq)) ? __ldg(res4 + base + (size_t)rr * rstep + wc) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
         };
         fetch_res(0, half);
@@ -518,7 +532,7 @@ __global__ void __launch_bounds__(kTcThreadsP, 1) conv1d_c4_tc_kernel(const __gr
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
                         const int rr = 4 * i + wr;
-                        if (q_base + rr >= a.Tq) continue;
+                        if (q_base + rr >= (RG ? it.rows : a.Tq)) continue;
                         float4 o = tile[rr * 8 + (wc ^ (rr & 7))];
                         float4 *dst = out4 + base + (size_t)rr * rstep + wc;
                         if (accumulate) {                            // same thread wrote *dst in the item before (chain-ordered lists)
@@ -689,9 +703,9 @@ bool tc_supported(const TcWeights &w, const ConvArgs &a) {
            (a.ups_u == 0 || a.Cout % 32 == 0) && a.Cout <= 3072;
 }
 
-template <int MODE, bool ST>
+template <int MODE, bool ST, bool RG = false>
 static int launch_mode(const TcArgs &p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = conv1d_c4_tc_kernel<MODE, ST>;
+    auto kern = conv1d_c4_tc_kernel<MODE, ST, RG>;
     // function attributes are per device: one process may drive several GPUs (the reference's mp.spawn gives one each,
     // but nothing in the C ABI forbids a handle per device in one process)
     static size_t configured[kMaxDevices] = {};
@@ -844,6 +858,13 @@ static int tc_plan(int n, const TcWeights *const *w, const ConvArgs *a, int prec
 static int tc_dispatch(TcArgs &p, int precision, int grid, size_t smem, cudaStream_t st) {
     const ConvArgs &a = p.a;
     const bool want_stats = getenv("SVB_TC_STATS") != nullptr;
+    if (a.rows) {                                                    // ragged batch
+        switch (precision) {
+            case SVB_PREC_TF32: return launch_mode<SVB_PREC_TF32, false, true>(p, grid, smem, st);
+            case SVB_PREC_TF32X3: return launch_mode<SVB_PREC_TF32X3, false, true>(p, grid, smem, st);
+            default: return launch_mode<SVB_PREC_BF16X3, false, true>(p, grid, smem, st);
+        }
+    }
     if ((want_stats || p.dbg != 0 || !p.collect) && precision == SVB_PREC_BF16X3) {
         // diagnostics: run the instrumented instantiation, wait for it and print where each role was blocked
         const size_t n = (size_t)grid * kTcStatSlots;
@@ -895,6 +916,7 @@ int launch_conv_tc(const TcWeights &w, const ConvArgs &a, int precision, cudaStr
             s.in = a.in + (size_t)b0 * c4t_groups(a.Cin) * a.in_Tp * 32;
             s.out = a.out + (size_t)b0 * c4t_groups(a.Cout) * a.out_Tp * 32;
             if (a.res) s.res = a.res + (size_t)b0 * c4t_groups(a.Cout) * a.out_Tp * 32;
+            if (a.rows) s.rows = a.rows + b0;
             SVB_TRY(launch_conv_tc(w, s, precision, st, max_ctas));
         }
         return SVB_OK;
@@ -903,9 +925,14 @@ int launch_conv_tc(const TcWeights &w, const ConvArgs &a, int precision, cudaStr
 }
 
 // whether `n` layers of this shape class fit one merged launch: the per-CTA item list lives in shared memory
-bool tc_merge_fits(int n, int B, int Tq, int Cout, int n_tile) {
-    const int tiles = (Tq + kTcM - 1) / kTcM, groups = (tiles + 1) / 2 * B * std::max(1, Cout / std::max(1, n_tile));
-    return (long long)groups * n <= (long long)(kMaxItems * 8 / 10) * sm_count();
+bool tc_merge_fits(int n, int B, int Tq, int Cout, int n_tile, const int *rows) {
+    long long groups = 0;
+    for (int b = 0; b < B; ++b) {
+        const int tiles = ((rows ? rows[b] : Tq) + kTcM - 1) / kTcM;
+        groups += (tiles + 1) / 2;
+    }
+    groups *= std::max(1, Cout / std::max(1, n_tile));
+    return groups * n <= (long long)(kMaxItems * 8 / 10) * sm_count();
 }
 
 // ---- merged launches: several layers of one shape class, host-built balanced work list
@@ -917,8 +944,7 @@ void tc_worklist_free(TcWorkList *wl) {
 
 // The schedule itself is plain host code (no CUDA call): exposed for the CPU tests through svb_tc_schedule_probe.
 int tc_schedule(int n, const int *KS, const int *has_res, const int *accum, int Cin, int B, int Tq, int MT, int col_blocks, bool chain_ordered,
-                int grid, std::vector<int4> *items_out, std::vector<int> *off_out, double *balance_out) {
-    const int tiles = (Tq + kTcM - 1) / kTcM;
+                int grid, std::vector<int4> *items_out, std::vector<int> *off_out, double *balance_out, const int *rows) {
     // cost of an item in "taps of one tile": the MMA work plus a constant for the memory-bound part (slab, epilogue)
     const double beta = 160.0 / std::max(32, Cin);
     struct Unit {
@@ -933,7 +959,8 @@ int tc_schedule(int n, const int *KS, const int *has_res, const int *accum, int 
     };
     std::vector<Unit> units;
     for (int nblk = 0; nblk < col_blocks; ++nblk)
-        for (int b = 0; b < B; ++b)
+        for (int b = 0; b < B; ++b) {
+            const int tiles = ((rows ? rows[b] : Tq) + kTcM - 1) / kTcM;       // a ragged clip: its own tile count
             for (int t = 0; t < tiles; t += MT) {
                 const int mt = std::min(MT, tiles - t);
                 if (chain_ordered) {
@@ -942,6 +969,7 @@ int tc_schedule(int n, const int *KS, const int *has_res, const int *accum, int 
                     for (int l = 0; l < n; ++l) units.push_back({unit_cost(l, mt), nblk, b, t * kTcM, mt, l});
                 }
             }
+        }
     // longest processing time first onto the least-loaded CTA.  Experiment kept behind SVB_TC_SPLIT=1: when the units are
     // too coarse for the 148 SMs (a few per CTA), split the cheapest two-tile units into one-tile halves and redo the
     // schedule.  Measured (same box): nominal balance 0.865 -> 0.95-0.99 but the forward gets 2 % SLOWER (4.66 -> 4.75 ms):
@@ -1015,7 +1043,7 @@ int tc_schedule(int n, const int *KS, const int *has_res, const int *accum, int 
         for (int u : mine[c]) {
             const Unit &U = units[u];
             for (int l = (U.layer < 0 ? 0 : U.layer); l < (U.layer < 0 ? n : U.layer + 1); ++l)
-                items.push_back(make_int4(l | (U.nblk << 8) | (U.mt << 24), U.b, U.t0, 0));
+                items.push_back(make_int4(l | (U.nblk << 8) | (U.mt << 24), U.b, U.t0, rows ? rows[U.b] : Tq));
         }
         off[c + 1] = (int)items.size();
         SVB_CHECK(off[c + 1] - off[c] <= kMaxItems, SVB_ERR_INVALID, "tc conv: %d work items on one CTA (limit %d)", off[c + 1] - off[c], kMaxItems);
@@ -1024,7 +1052,8 @@ int tc_schedule(int n, const int *KS, const int *has_res, const int *accum, int 
     return SVB_OK;
 }
 
-int tc_worklist_build(int n, const TcWeights *const *w, const ConvArgs *a, int precision, bool chain_ordered, TcWorkList *out) {
+int tc_worklist_build(int n, const TcWeights *const *w, const ConvArgs *a, int precision, bool chain_ordered, TcWorkList *out,
+                      const int *rows, cudaStream_t st) {
     TcArgs p;
     size_t smem = 0;
     SVB_TRY(tc_plan(n, w, a, precision, p, smem));
@@ -1034,13 +1063,23 @@ int tc_worklist_build(int n, const TcWeights *const *w, const ConvArgs *a, int p
     std::vector<int4> items;
     std::vector<int> off;
     double balance = 0;
-    SVB_TRY(tc_schedule(n, KS, has_res, accum, a[0].Cin, a[0].B, a[0].Tq, p.MT, p.col_blocks, chain_ordered, grid, &items, &off, &balance));
-    tc_worklist_free(out);
-    SVB_CUDA(cudaMalloc((void **)&out->items, std::max<size_t>(items.size(), 1) * sizeof(int4)));
-    SVB_CUDA(cudaMalloc((void **)&out->off, off.size() * sizeof(int)));
-    SVB_CUDA(cudaMemcpy(out->items, items.data(), items.size() * sizeof(int4), cudaMemcpyHostToDevice));
-    SVB_CUDA(cudaMemcpy(out->off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice));
+    SVB_TRY(tc_schedule(n, KS, has_res, accum, a[0].Cin, a[0].B, a[0].Tq, p.MT, p.col_blocks, chain_ordered, grid, &items, &off, &balance,
+                        rows));
+    // grow-only device buffers, stream-ordered upload: a ragged batch rebuilds its lists on every call with new lengths,
+    // and cudaFree would synchronise the device each time
+    if (items.size() > out->cap_items || off.size() > out->cap_off) {
+        if (out->items) SVB_CUDA(cudaFree(out->items));
+        if (out->off) SVB_CUDA(cudaFree(out->off));
+        out->items = nullptr, out->off = nullptr;
+        out->cap_items = std::max<size_t>(items.size(), 1) * 5 / 4, out->cap_off = off.size();
+        SVB_CUDA(cudaMalloc((void **)&out->items, out->cap_items * sizeof(int4)));
+        SVB_CUDA(cudaMalloc((void **)&out->off, out->cap_off * sizeof(int)));
+    }
+    // from pageable memory: the runtime stages the bytes before returning, so the vectors may go out of scope
+    SVB_CUDA(cudaMemcpyAsync(out->items, items.data(), items.size() * sizeof(int4), cudaMemcpyHostToDevice, st));
+    SVB_CUDA(cudaMemcpyAsync(out->off, off.data(), off.size() * sizeof(int), cudaMemcpyHostToDevice, st));
     out->grid = grid, out->n_items = (int)items.size(), out->MT = p.MT, out->n_layers = n, out->chain_ordered = chain_ordered;
+    out->valid = true;
     if (getenv("SVB_TC_VERBOSE"))
         fprintf(stderr, "[tc] work list: %d layers, %zu items over %d CTAs, balance %.3f (mean / max load)\n", n, items.size(), grid, balance);
     return SVB_OK;
@@ -1051,7 +1090,7 @@ int launch_conv_tc_multi(int n, const TcWeights *const *w, const ConvArgs *a, in
     TcArgs p;
     size_t smem = 0;
     SVB_TRY(tc_plan(n, w, a, precision, p, smem));
-    SVB_CHECK(wl.items && wl.n_layers == n && wl.MT == p.MT && wl.grid == sm_count(), SVB_ERR_STATE,
+    SVB_CHECK(wl.valid && wl.n_layers == n && wl.MT == p.MT && wl.grid == sm_count(), SVB_ERR_STATE,
               "tc conv: work list was built for another plan (layers %d / %d, MT %d / %d)", wl.n_layers, n, wl.MT, p.MT);
     p.work = wl.items, p.work_off = wl.off;
     return tc_dispatch(p, precision, wl.grid, smem, st);
@@ -1071,8 +1110,37 @@ extern "C" int64_t svb_tc_schedule_probe(int32_t n_layers, const int32_t *KS, co
     std::vector<int> off;
     int ks[svb::kTcMaxLayers], hr[svb::kTcMaxLayers], ac[svb::kTcMaxLayers];
     for (int l = 0; l < n_layers; ++l) ks[l] = KS[l], hr[l] = has_res[l], ac[l] = accumulate[l];
-    SVB_TRY(svb::tc_schedule(n_layers, ks, hr, ac, Cin, B, Tq, MT, col_blocks, chain_ordered != 0, grid, &items, &off, balance_out));
+    SVB_TRY(svb::tc_schedule(n_layers, ks, hr, ac, Cin, B, Tq, MT, col_blocks, chain_ordered != 0, grid, &items, &off, balance_out, nullptr));
     SVB_CHECK((int64_t)items.size() <= items_capacity, SVB_ERR_INVALID, "tc_schedule_probe: %zu items, capacity %lld", items.size(),
+              (long long)items_capacity);
+    for (size_t i = 0; i < items.size(); ++i) {
+        int32_t *o = items_out + 5 * i;                             // layer, column block, clip, first row, tiles
+        o[0] = items[i].x & 0xff, o[1] = (items[i].x >> 8) & 0xffff, o[2] = items[i].y, o[3] = items[i].z, o[4] = items[i].x >> 24;
+    }
+    for (int c = 0; c <= grid; ++c) off_out[c] = off[c];
+    return (int64_t)items.size();
+}
+
+// The same view for a ragged batch: clip b has rows_per_clip[b] rows (1 <= rows <= Tq).
+extern "C" int64_t svb_tc_schedule_probe_ragged(int32_t n_layers, const int32_t *KS, const int32_t *has_res, const int32_t *accumulate,
+                                                int32_t Cin, int32_t B, const int32_t *rows_per_clip, int32_t MT, int32_t col_blocks,
+                                                int32_t chain_ordered, int32_t grid, int32_t *items_out, int64_t items_capacity,
+                                                int32_t *off_out, double *balance_out) {
+    SVB_CHECK(n_layers >= 1 && n_layers <= svb::kTcMaxLayers && KS && has_res && accumulate && B > 0 && rows_per_clip && (MT == 1 || MT == 2) &&
+                  col_blocks >= 1 && grid >= 1 && items_out && off_out && balance_out,
+              SVB_ERR_INVALID, "tc_schedule_probe_ragged: bad argument");
+    int Tq = 0;
+    for (int b = 0; b < B; ++b) {
+        SVB_CHECK(rows_per_clip[b] >= 1, SVB_ERR_INVALID, "tc_schedule_probe_ragged: clip %d has %d rows", b, rows_per_clip[b]);
+        Tq = std::max(Tq, (int)rows_per_clip[b]);
+    }
+    std::vector<int4> items;
+    std::vector<int> off;
+    int ks[svb::kTcMaxLayers], hr[svb::kTcMaxLayers], ac[svb::kTcMaxLayers];
+    for (int l = 0; l < n_layers; ++l) ks[l] = KS[l], hr[l] = has_res[l], ac[l] = accumulate[l];
+    const std::vector<int> rows(rows_per_clip, rows_per_clip + B);
+    SVB_TRY(svb::tc_schedule(n_layers, ks, hr, ac, Cin, B, Tq, MT, col_blocks, chain_ordered != 0, grid, &items, &off, balance_out, rows.data()));
+    SVB_CHECK((int64_t)items.size() <= items_capacity, SVB_ERR_INVALID, "tc_schedule_probe_ragged: %zu items, capacity %lld", items.size(),
               (long long)items_capacity);
     for (size_t i = 0; i < items.size(); ++i) {
         int32_t *o = items_out + 5 * i;                             // layer, column block, clip, first row, tiles

@@ -33,11 +33,15 @@ struct TcWorkList {
     int *off = nullptr;
     int grid = 0, n_items = 0, MT = 0, n_layers = 0;
     bool chain_ordered = false;
+    bool valid = false;             // false: rebuild before the next launch (the buffers are kept and only grow)
+    size_t cap_items = 0, cap_off = 0;
 };
-int tc_worklist_build(int n, const TcWeights *const *w, const ConvArgs *a, int precision, bool chain_ordered, TcWorkList *out);
+// rows: host [B] valid GEMM rows per clip of a ragged batch (nullptr: every clip a[0].Tq); the list is uploaded on `st`
+int tc_worklist_build(int n, const TcWeights *const *w, const ConvArgs *a, int precision, bool chain_ordered, TcWorkList *out,
+                      const int *rows = nullptr, cudaStream_t st = 0);
 void tc_worklist_free(TcWorkList *wl);
 // the per-CTA item list of a merged launch is bounded (shared memory): very long batches fall back to one launch per layer
-bool tc_merge_fits(int n, int B, int Tq, int Cout, int n_tile);
+bool tc_merge_fits(int n, int B, int Tq, int Cout, int n_tile, const int *rows = nullptr);
 // one persistent launch over `n` layers that share channels / rows / upsampling (taps, dilation and pointers may differ)
 int launch_conv_tc_multi(int n, const TcWeights *const *w, const ConvArgs *a, int precision, cudaStream_t st, const TcWorkList &wl);
 // max_ctas > 0 caps the persistent grid (used to run independent ResBlock chains side by side on SM subsets)

@@ -134,20 +134,31 @@ struct ProfScope {
     }
 };
 
+// valid GEMM rows of a layer with Tq rows per clip at the longest clip (= B * Tq for a uniform batch)
+double valid_rows_total(const svb_gen *g, int Tq) { return g->cur_frames * (double)(Tq / g->cur_T); }
+// host [B] valid rows per clip at Tq rows for the longest clip; empty for a uniform batch
+std::vector<int> clip_rows(const svb_gen *g, int Tq) {
+    std::vector<int> r(g->cur_len);
+    for (int &v : r) v *= Tq / g->cur_T;
+    return r;
+}
+
 int run_conv(svb_gen *g, const ConvLayer &L, const float *in, int in_Tp, float *out, int out_Tp, const float *res,
              int B, int Tq, float in_slope, float scale, int accumulate, cudaStream_t st, int max_ctas = 0) {
+    const double rows = valid_rows_total(g, Tq);
     g->last_launches += 1;
-    g->last_flops += 2.0 * L.macs_per_row * (double)B * Tq;
+    g->last_flops += 2.0 * L.macs_per_row * rows;
     const bool tc = g->cfg.precision != SVB_PREC_FP32 && L.tc.ok;
-    const double rows_out = (double)B * Tq * (L.ups_u > 0 ? L.ups_u : 1);
+    const double rows_out = rows * (L.ups_u > 0 ? L.ups_u : 1);
     // layer-streaming bytes (SURVEY 8(d)): input once, output once, residual / accumulated sum once more each
-    const double bytes = 4.0 * ((double)B * Tq * L.Cin + rows_out * L.Cout * (1 + (res ? 1 : 0) + (accumulate ? 1 : 0)));
+    const double bytes = 4.0 * (rows * L.Cin + rows_out * L.Cout * (1 + (res ? 1 : 0) + (accumulate ? 1 : 0)));
     ProfScope ps(g, st, tc ? (L.ups_u ? "conv1d_c4_tc (upsampler)" : "conv1d_c4_tc (resblock)") : "conv1d_c4_ffma", bytes,
-                 2.0 * L.macs_per_row * (double)B * Tq);
+                 2.0 * L.macs_per_row * rows);
     ConvArgs a;
     a.in = in, a.w = L.w, a.bias = L.b, a.res = res, a.out = out;
     a.B = B, a.Cin = L.Cin, a.in_Tp = in_Tp, a.Cout = L.Cout, a.out_Tp = out_Tp, a.CoutP = L.CoutP, a.Tq = Tq;
     a.KS = L.KS, a.dil = L.dil, a.ups_u = L.ups_u, a.in_slope = in_slope, a.out_scale = scale, a.accumulate = accumulate;
+    a.rows = g->cur_len_dev, a.rows_mul = Tq / g->cur_T;
     if (g->cfg.precision != SVB_PREC_FP32 && tc_supported(L.tc, a)) return launch_conv_tc(L.tc, a, g->cfg.precision, st, max_ctas);
     return launch_conv_ffma(a, st);
 }
@@ -160,14 +171,16 @@ int run_conv_multi(svb_gen *g, int stage, int nk, const ConvLayer *const *Ls, co
     ConvArgs a[kTcMaxLayers];
     const TcWeights *w[kTcMaxLayers];
     double bytes = 0, flops = 0;
+    const double rows = valid_rows_total(g, Tq);
     for (int j = 0; j < nk; ++j) {
         const ConvLayer &L = *Ls[j];
         a[j].in = in[j], a[j].w = L.w, a[j].bias = L.b, a[j].res = res[j], a[j].out = out[j];
         a[j].B = B, a[j].Cin = L.Cin, a[j].in_Tp = Tp, a[j].Cout = L.Cout, a[j].out_Tp = Tp, a[j].CoutP = L.CoutP, a[j].Tq = Tq;
         a[j].KS = L.KS, a[j].dil = L.dil, a[j].ups_u = 0, a[j].in_slope = in_slope, a[j].out_scale = scale[j], a[j].accumulate = accumulate[j];
+        a[j].rows = g->cur_len_dev, a[j].rows_mul = Tq / g->cur_T;
         w[j] = &L.tc;
-        bytes += 4.0 * ((double)B * Tq * L.Cin + (double)B * Tq * L.Cout * (1 + (res[j] ? 1 : 0) + (accumulate[j] ? 1 : 0)));
-        flops += 2.0 * L.macs_per_row * (double)B * Tq;
+        bytes += 4.0 * (rows * L.Cin + rows * L.Cout * (1 + (res[j] ? 1 : 0) + (accumulate[j] ? 1 : 0)));
+        flops += 2.0 * L.macs_per_row * rows;
     }
     g->last_launches += 1;
     g->last_flops += flops;
@@ -176,7 +189,10 @@ int run_conv_multi(svb_gen *g, int stage, int nk, const ConvLayer *const *Ls, co
     for (int attempt = 0; attempt < 2; ++attempt) {
         const int key = stage * 4 + (chain_ordered ? 2 : 0) + attempt;
         TcWorkList &wl = g->worklists[key];
-        if (!wl.items) SVB_TRY(tc_worklist_build(nk, w, a, g->cfg.precision, chain_ordered, &wl));
+        if (!wl.valid) {
+            const std::vector<int> rh = clip_rows(g, Tq);
+            SVB_TRY(tc_worklist_build(nk, w, a, g->cfg.precision, chain_ordered, &wl, rh.empty() ? nullptr : rh.data(), st));
+        }
         const int rc = launch_conv_tc_multi(nk, w, a, g->cfg.precision, st, wl);
         if (rc != SVB_ERR_STATE) return rc;
     }
@@ -184,14 +200,21 @@ int run_conv_multi(svb_gen *g, int stage, int nk, const ConvLayer *const *Ls, co
     return SVB_ERR_STATE;
 }
 
+// The one generator forward.  lens == nullptr: B clips of T frames.  lens = host [B] (1 <= lens[b] <= T): a ragged batch in the
+// padded layout (clip b's frames 0 .. lens[b] - 1; nothing past them is read, wav past lens[b] * hop is written as 0), or, with
+// `packed`, clip after clip in mel [sum lens, n_mel] (frame-major) / f0 [sum lens] / wav [sum lens * hop].
 int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float *f0, const float *rand_ini,
-                 const float *noise, uint64_t seed, int B, int T, float *wav, cudaStream_t st) {
+                 const float *noise, uint64_t seed, int B, int T, float *wav, cudaStream_t st, const int32_t *lens = nullptr,
+                 bool packed = false) {
     SVB_CHECK(g && g->finalized, SVB_ERR_STATE, "generator: forward before finalize");
     SVB_CHECK(!g->dirty, SVB_ERR_STATE, "generator: weights were set after finalize; call svb_gen_update_weights first");
     SVB_CHECK(mel && wav && B > 0 && T > 0, SVB_ERR_INVALID, "generator: null buffer or empty batch (B %d T %d)", B, T);
     SVB_CHECK(!f0 || g->cfg.use_pitch_embed, SVB_ERR_INVALID, "generator: f0 given but use_pitch_embed is off");
     SVB_CHECK((rand_ini == nullptr) == (noise == nullptr), SVB_ERR_INVALID,
               "generator: rand_ini and noise must be given together");
+    SVB_CHECK(!lens || !g->training, SVB_ERR_INVALID,
+              "generator: a ragged batch is inference only (training takes clips of equal length)");
+    SVB_CHECK(!packed || (lens && mel_frame_major && !noise), SVB_ERR_INVALID, "generator: bad packed-layout call");
     SVB_CUDA(cudaSetDevice(g->device));
     size_t need = 0;
     Buffers bf = plan_workspace(g, B, T, &need);
@@ -201,14 +224,41 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
         SVB_CUDA(cudaMalloc((void **)&g->ws, need));
         g->ws_cap = need, g->ws_B = 0;
     }
-    if (g->ws_B != B || g->ws_T != T) {
-        for (auto &kv : g->worklists) tc_worklist_free(&kv.second);
-        g->worklists.clear();
+    std::vector<int> len;
+    if (lens) len.assign(lens, lens + B);
+    if (g->ws_B != B || g->ws_T != T || len != g->wl_len) {            // the work lists depend on the batch and its lengths
+        for (auto &kv : g->worklists) kv.second.valid = false;
+        g->wl_len = len;
     }
     if (g->ws_B != B || g->ws_T != T || g->ws_training != g->training) {   // new layout: rebuild the zero padding of every buffer
         SVB_CUDA(cudaMemsetAsync(g->ws, 0, need, st));
         g->ws_B = B, g->ws_T = T, g->ws_training = g->training;
+        g->hw.assign(B, 0);
     }
+    g->cur_len = len, g->cur_len_dev = nullptr, g->cur_T = T, g->cur_frames = (double)B * T;
+    Ragged rg;
+    int stale_rows = 0;                         // longest stale tail (frames) a shrunk clip left behind
+    if (lens) {
+        // device table [len B | hw B | off B + 1], grow-only; uploaded from pageable memory (staged before the call returns)
+        std::vector<int> tab(3 * (size_t)B + 1);
+        double frames = 0;
+        for (int b = 0; b < B; ++b) {
+            tab[b] = len[b], tab[B + b] = g->hw[b], tab[2 * B + b] = (int)frames;
+            stale_rows = std::max(stale_rows, g->hw[b] - len[b]);
+            frames += len[b];
+        }
+        tab[3 * B] = (int)frames;
+        if (tab.size() > g->rg_cap) {
+            if (g->rg_dev) SVB_CUDA(cudaFree(g->rg_dev));
+            g->rg_dev = nullptr, g->rg_cap = 0;
+            SVB_CUDA(cudaMalloc((void **)&g->rg_dev, tab.size() * sizeof(int)));
+            g->rg_cap = tab.size();
+        }
+        SVB_CUDA(cudaMemcpyAsync(g->rg_dev, tab.data(), tab.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+        g->cur_len_dev = g->rg_dev, g->cur_frames = frames;
+        rg.len = g->rg_dev, rg.off = packed ? g->rg_dev + 2 * B : nullptr;
+    }
+    for (int b = 0; b < B; ++b) g->hw[b] = lens ? len[b] : T;
     g->bf = bf, g->last_T = T, g->last_nsf = f0 != nullptr;
     g->last_launches = 0, g->last_flops = 0, g->last_B = B;
     g->taps.clear();
@@ -218,10 +268,35 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
     auto F = [&](size_t off) { return reinterpret_cast<float *>(g->ws + off); };
     const int n_mel = g->cfg.n_mel, C0 = g->cfg.upsample_initial_channel;
     const int Tp0 = c4t_rows(T);
+    const double frames = g->cur_frames;
+    if (stale_rows > 0) {
+        // a clip shrank since the last forward: its rows [len, hw) of every buffer a conv reads past the clip's end
+        // go back to zero (the mel buffer is rewritten in full below)
+        std::vector<ZeroSeg> segs;
+        segs.push_back({F(bf.pre), c4t_groups(C0), Tp0, 1});
+        int mul = 1, max_rows = stale_rows;
+        for (size_t i = 0; i < g->stages.size(); ++i) {
+            const Stage &s = g->stages[i];
+            mul *= s.u;
+            const int Tip = c4t_rows(T * mul), gr = c4t_groups(s.C);
+            std::vector<size_t> offs = {bf.X[i], bf.S[i]};
+            for (auto &v : bf.A[i]) offs.insert(offs.end(), v.begin(), v.end());
+            for (auto &v : bf.R[i]) offs.insert(offs.end(), v.begin(), v.end());
+            std::sort(offs.begin(), offs.end());
+            offs.erase(std::unique(offs.begin(), offs.end()), offs.end());
+            for (size_t o : offs) segs.push_back({F(o), gr, Tip, mul});
+            max_rows = std::max(max_rows, stale_rows * mul);
+        }
+        ProfScope ps(g, st, "zero stale rows", 0, 0);
+        for (size_t i0 = 0; i0 < segs.size(); i0 += kMaxZeroSegs)
+            SVB_TRY(launch_zero_tails(segs.data() + i0, (int)std::min<size_t>(kMaxZeroSegs, segs.size() - i0), B, g->rg_dev,
+                                      g->rg_dev + B, max_rows, st));
+        g->last_launches += (int64_t)((segs.size() + kMaxZeroSegs - 1) / kMaxZeroSegs);
+    }
     {
-        ProfScope ps(g, st, "mel layout", 8.0 * B * n_mel * T, 0);
-        if (mel_frame_major) SVB_TRY(launch_btc_to_c4t(mel, F(bf.mel), B, n_mel, T, Tp0, st));
-        else SVB_TRY(launch_nct_to_c4t(mel, F(bf.mel), B, n_mel, T, Tp0, st));
+        ProfScope ps(g, st, "mel layout", 8.0 * n_mel * frames, 0);
+        if (mel_frame_major) SVB_TRY(launch_btc_to_c4t(mel, F(bf.mel), B, n_mel, T, Tp0, st, rg));
+        else SVB_TRY(launch_nct_to_c4t(mel, F(bf.mel), B, n_mel, T, Tp0, st, rg));
     }
     g->last_launches += 1;
 
@@ -240,9 +315,10 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
         }
         int l = 0;
         {
-            ProfScope ps(g, ns, "nsf source (4 kernels)", 4.0 * B * (T + (double)Tw * (noise ? 10 : 1)), 60.0 * B * Tw * 9);
+            const double samples = frames * g->hop;
+            ProfScope ps(g, ns, "nsf source (4 kernels)", 4.0 * (frames + samples * (noise ? 10 : 1)), 60.0 * samples * 9);
             SVB_TRY(launch_nsf_source(f0, rand_ini, noise, seed, B, T, g->hop, (float)g->cfg.audio_sample_rate, g->lin_w,
-                                      g->lin_b_dev, g->ws + bf.nsf, har, g->training ? F(bf.sines) : nullptr, ns, &l));
+                                      g->lin_b_dev, g->ws + bf.nsf, har, g->training ? F(bf.sines) : nullptr, ns, &l, rg.len, rg.off));
         }
         if (har_on_side) SVB_CUDA(cudaEventRecord(g->ev_chain[0], ns));
         g->last_launches += l;
@@ -263,11 +339,12 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
         SVB_TRY(run_conv(g, s.up, x_in, Tin_p, X, Tip, nullptr, B, Tin, 0.1f, 1.f, 0, st));
         if (f0) {                                   // x = x + noise_convs[i](har_source)   :155-157
             if (har_on_side && i == 0) SVB_CUDA(cudaStreamWaitEvent(st, g->ev_chain[0], 0));
-            ProfScope ps(g, st, "noise_conv_add", 4.0 * B * (2.0 * Ti * s.C + Tw), 2.0 * B * (double)Ti * s.C * s.noise.K);
+            const double rows = valid_rows_total(g, Ti);
+            ProfScope ps(g, st, "noise_conv_add", 4.0 * (2.0 * rows * s.C + frames * g->hop), 2.0 * rows * s.C * s.noise.K);
             SVB_TRY(launch_noise_conv_add(X, B, s.C, Ti, Tip, har, Tw, s.noise.w, s.noise.b, s.noise.K, s.noise.stride,
-                                          s.noise.pad, st));
+                                          s.noise.pad, st, rg, Ti / T, g->hop));
             g->last_launches += 1;
-            g->last_flops += 2.0 * B * (double)Ti * s.C * s.noise.K;
+            g->last_flops += 2.0 * rows * s.C * s.noise.K;
         }
         g->taps["ups" + std::to_string(i)] = Tap{X, s.C, Ti, Tip, false};
         // xs = sum_j resblocks[i*nk + j](x) ; x = xs / nk      :158-164
@@ -278,7 +355,11 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
         const int sms = 148;
         // merged schedule: step m of all nk chains in ONE persistent launch (the chains only share their input)
         bool merged = g->merge && !par && nk > 1 && nk <= kTcMaxLayers && g->cfg.precision != SVB_PREC_FP32 &&
-                      s.c1[0][0].tc.ok && tc_merge_fits(nk, B, Ti, s.C, s.c1[0][0].tc.n_tile);
+                      s.c1[0][0].tc.ok;
+        if (merged) {
+            const std::vector<int> rh = clip_rows(g, Ti);
+            merged = tc_merge_fits(nk, B, Ti, s.C, s.c1[0][0].tc.n_tile, rh.empty() ? nullptr : rh.data());
+        }
         for (int j = 0; merged && j < nk; ++j)
             for (int m = 0; m < nd; ++m) {
                 ConvArgs probe;
@@ -358,11 +439,13 @@ int forward_impl(svb_gen *g, const float *mel, bool mel_frame_major, const float
     }
     // x = tanh(conv_post(leaky_relu(x)))   default slope 0.01   :165-167
     {
-        ProfScope ps(g, st, "conv_post_tanh", 4.0 * B * Tin * (g->post_C + 1.0), 2.0 * B * (double)Tin * g->post_C * g->post_K);
-        SVB_TRY(launch_conv_post_tanh(x_in, B, g->post_C, Tin, Tin_p, g->post_wq, g->post_b_dev, g->post_K, 0.01f, wav, st));
+        const double rows = valid_rows_total(g, Tin);
+        ProfScope ps(g, st, "conv_post_tanh", 4.0 * rows * (g->post_C + 1.0), 2.0 * rows * g->post_C * g->post_K);
+        SVB_TRY(launch_conv_post_tanh(x_in, B, g->post_C, Tin, Tin_p, g->post_wq, g->post_b_dev, g->post_K, 0.01f, wav, st, rg,
+                                      Tin / T));
     }
     g->last_launches += 1;
-    g->last_flops += 2.0 * B * (double)Tin * g->post_C * g->post_K;
+    g->last_flops += 2.0 * valid_rows_total(g, Tin) * g->post_C * g->post_K;
     if (g->training) SVB_CUDA(cudaMemcpyAsync(F(bf.wav), wav, (size_t)B * Tw * 4, cudaMemcpyDeviceToDevice, st));
     if (g->timing) SVB_CUDA(cudaEventRecord(g->ev1, st));
     return SVB_OK;
@@ -422,6 +505,7 @@ extern "C" void svb_gen_destroy(svb_gen_t *g) {
     for (void *p : g->dev_allocs) cudaFree(p);
     for (auto &kv : g->worklists) tc_worklist_free(&kv.second);
     if (g->ws) cudaFree(g->ws);
+    if (g->rg_dev) cudaFree(g->rg_dev);
     if (g->bws) cudaFree(g->bws);
     for (void *p : g->job_allocs) cudaFree(p);
     for (auto &kv : g->nat_dev) cudaFree(kv.second.p);
@@ -549,6 +633,31 @@ extern "C" int svb_gen_forward(svb_gen_t *g, const float *mel_dev, const float *
     return forward_impl(g, mel_dev, false, f0_dev, rand_ini_dev, noise_dev, seed, B, T, wav_dev, as_stream(stream));
 }
 
+namespace {
+// lengths of a ragged batch: every clip 1 .. T_max frames (T_max <= 0: no upper bound); checked before any CUDA call
+int check_lengths(const char *what, const int32_t *lens, int B, int T_max) {
+    SVB_CHECK(lens, SVB_ERR_INVALID, "%s: lengths is NULL", what);
+    SVB_CHECK(B > 0, SVB_ERR_INVALID, "%s: empty batch (B %d)", what, B);
+    long long frames = 0;
+    for (int b = 0; b < B; ++b) {
+        SVB_CHECK(lens[b] >= 1 && (T_max <= 0 || lens[b] <= T_max), SVB_ERR_INVALID,
+                  "%s: length %d of clip %d is outside [1, T_max %d]", what, lens[b], b, T_max);
+        frames += lens[b];
+    }
+    SVB_CHECK(frames < (1ll << 31) / 4096, SVB_ERR_INVALID, "%s: %lld frames in one batch", what, frames);
+    return SVB_OK;
+}
+}  // namespace
+
+extern "C" int svb_gen_forward_ragged(svb_gen_t *g, const float *mel_dev, const float *f0_dev, const int32_t *lengths_host,
+                                      const float *rand_ini_dev, const float *noise_dev, uint64_t seed, int32_t B, int32_t T_max,
+                                      float *wav_dev, void *stream) {
+    SVB_CHECK(T_max > 0, SVB_ERR_INVALID, "gen_forward_ragged: T_max %d", T_max);
+    SVB_TRY(check_lengths("gen_forward_ragged", lengths_host, B, T_max));
+    SVB_CHECK(g, SVB_ERR_INVALID, "gen_forward_ragged: null handle");
+    return forward_impl(g, mel_dev, false, f0_dev, rand_ini_dev, noise_dev, seed, B, T_max, wav_dev, as_stream(stream), lengths_host);
+}
+
 extern "C" int svb_gen_spec2wav_host(svb_gen_t *g, const float *mel_host, const float *f0_host, uint64_t seed, int32_t B,
                                      int32_t T, float *wav_host, void *stream) {
     SVB_CHECK(g && g->finalized, SVB_ERR_STATE, "spec2wav: generator not finalized");
@@ -587,31 +696,39 @@ extern "C" int svb_gen_spec2wav_host(svb_gen_t *g, const float *mel_host, const 
 // ---- save_wav's sample conversion on the device (utils/audio.py:11-16): [norm: wav / max|wav| per clip,] wav * 32767,
 // numpy's float -> int16 cast (truncation toward zero).  Done before the D2H copy, the transfer is 2 bytes per sample.
 namespace {
-__global__ void clip_absmax_kernel(const float *__restrict__ x, long long n, unsigned *__restrict__ mx) {
+// off [B + 1] (frames, optional): clip b is the packed range [off[b] * hop, off[b + 1] * hop) instead of [b * n, (b + 1) * n)
+__global__ void clip_absmax_kernel(const float *__restrict__ x, long long n, unsigned *__restrict__ mx, const int *__restrict__ off, int hop) {
     const int b = blockIdx.y;
+    const size_t base = off ? (size_t)off[b] * hop : (size_t)b * n;
+    if (off) n = (long long)(off[b + 1] - off[b]) * hop;
     float m = 0.f;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-        m = fmaxf(m, fabsf(x[(size_t)b * n + i]));
+        m = fmaxf(m, fabsf(x[base + i]));
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     if ((threadIdx.x & 31) == 0) atomicMax(mx + b, __float_as_uint(m));      // non-negative floats order like their bit patterns
 }
-__global__ void to_int16_kernel(const float *__restrict__ x, long long n, const unsigned *__restrict__ mx, int16_t *__restrict__ y) {
+__global__ void to_int16_kernel(const float *__restrict__ x, long long n, const unsigned *__restrict__ mx, int16_t *__restrict__ y,
+                                const int *__restrict__ off, int hop) {
     const int b = blockIdx.y;
+    const size_t base = off ? (size_t)off[b] * hop : (size_t)b * n;
+    if (off) n = (long long)(off[b + 1] - off[b]) * hop;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        float v = x[(size_t)b * n + i];
+        float v = x[base + i];
         if (mx) v = __fdiv_rn(v, __uint_as_float(mx[b]));
         v = __fmul_rn(v, 32767.f);
-        y[(size_t)b * n + i] = (int16_t)__float2int_rz(v);
+        y[base + i] = (int16_t)__float2int_rz(v);
     }
 }
-int wav_to_int16(const float *wav_dev, int B, long long n, int norm, int16_t *out_dev, unsigned *mx_dev, cudaStream_t st) {
+// n = samples per clip (with `off`: of the longest clip, sizes the grid)
+int wav_to_int16(const float *wav_dev, int B, long long n, int norm, int16_t *out_dev, unsigned *mx_dev, cudaStream_t st,
+                 const int *off = nullptr, int hop = 1) {
     const dim3 grid((unsigned)std::min<long long>((n + 255) / 256, 148 * 4), (unsigned)B);
     if (norm) {
         SVB_CUDA(cudaMemsetAsync(mx_dev, 0, (size_t)B * sizeof(unsigned), st));
-        clip_absmax_kernel<<<grid, 256, 0, st>>>(wav_dev, n, mx_dev);
+        clip_absmax_kernel<<<grid, 256, 0, st>>>(wav_dev, n, mx_dev, off, hop);
     }
-    to_int16_kernel<<<grid, 256, 0, st>>>(wav_dev, n, norm ? mx_dev : nullptr, out_dev);
+    to_int16_kernel<<<grid, 256, 0, st>>>(wav_dev, n, norm ? mx_dev : nullptr, out_dev, off, hop);
     SVB_CUDA(cudaGetLastError());
     return SVB_OK;
 }
@@ -670,6 +787,73 @@ extern "C" int svb_gen_spec2wav_host_i16(svb_gen_t *g, const float *mel_host, co
     SVB_CUDA(cudaStreamSynchronize(st));
     memcpy(wav_host, g->pin_out, n_out * 2);
     return SVB_OK;
+}
+
+// ---- spec2wav over a ragged batch from host memory (packed clip after clip, svb_wav2spec_batch_host's convention):
+// one H2D of mel + f0, the forward reads the packed rows directly (layout kernel / NSF source) and conv_post writes the packed
+// waveform, [int16 conversion with a per-clip peak,] one D2H.
+namespace {
+int spec2wav_ragged(svb_gen_t *g, const char *what, const float *mel_host, const float *f0_host, const int32_t *lens, int B,
+                    uint64_t seed, bool i16, int norm, void *wav_host, void *stream) {
+    SVB_CHECK(mel_host && wav_host, SVB_ERR_INVALID, "%s: null buffer", what);
+    SVB_TRY(check_lengths(what, lens, B, 0));
+    SVB_CHECK(g && g->finalized, SVB_ERR_STATE, "%s: generator not finalized", what);
+    SVB_CHECK(!i16 || B <= 4096, SVB_ERR_INVALID, "%s: batch %d > 4096", what, B);
+    int T_max = 0;
+    size_t frames = 0;
+    for (int b = 0; b < B; ++b) T_max = std::max(T_max, (int)lens[b]), frames += lens[b];
+    SVB_CUDA(cudaSetDevice(g->device));
+    cudaStream_t st = as_stream(stream);
+    const size_t n_mel = frames * g->cfg.n_mel, n_f0 = f0_host ? frames : 0;
+    const size_t n_in = n_mel + n_f0, n_out = frames * g->hop;
+    if (n_in > g->pin_in_cap) {
+        if (g->pin_in) cudaFreeHost(g->pin_in);
+        if (g->dev_in) cudaFree(g->dev_in);
+        g->pin_in = nullptr, g->dev_in = nullptr, g->pin_in_cap = 0;
+        SVB_CUDA(cudaMallocHost((void **)&g->pin_in, n_in * 4));
+        SVB_CUDA(cudaMalloc((void **)&g->dev_in, n_in * 4));
+        g->pin_in_cap = n_in;
+    }
+    if (n_out > g->pin_out_cap) {
+        if (g->pin_out) cudaFreeHost(g->pin_out);
+        if (g->dev_out) cudaFree(g->dev_out);
+        g->pin_out = nullptr, g->dev_out = nullptr, g->pin_out_cap = 0;
+        SVB_CUDA(cudaMallocHost((void **)&g->pin_out, n_out * 4));
+        SVB_CUDA(cudaMalloc((void **)&g->dev_out, n_out * 4));
+        g->pin_out_cap = n_out;
+    }
+    if (i16 && n_out > g->i16_cap) {
+        if (g->dev_i16) cudaFree(g->dev_i16);
+        g->dev_i16 = nullptr, g->i16_cap = 0;
+        SVB_CUDA(cudaMalloc((void **)&g->dev_i16, n_out * 2 + (size_t)4096 * sizeof(unsigned)));
+        g->i16_cap = n_out;
+    }
+    memcpy(g->pin_in, mel_host, n_mel * 4);
+    if (f0_host) memcpy(g->pin_in + n_mel, f0_host, n_f0 * 4);
+    SVB_CUDA(cudaMemcpyAsync(g->dev_in, g->pin_in, n_in * 4, cudaMemcpyHostToDevice, st));
+    SVB_TRY(forward_impl(g, g->dev_in, true, f0_host ? g->dev_in + n_mel : nullptr, nullptr, nullptr, seed, B, T_max, g->dev_out, st,
+                         lens, true));
+    if (i16) {
+        unsigned *mx = reinterpret_cast<unsigned *>(reinterpret_cast<char *>(g->dev_i16) + (g->i16_cap * 2 + 3) / 4 * 4);
+        SVB_TRY(wav_to_int16(g->dev_out, B, (long long)T_max * g->hop, norm, g->dev_i16, mx, st, g->rg_dev + 2 * B, g->hop));
+        SVB_CUDA(cudaMemcpyAsync(g->pin_out, g->dev_i16, n_out * 2, cudaMemcpyDeviceToHost, st));
+    } else {
+        SVB_CUDA(cudaMemcpyAsync(g->pin_out, g->dev_out, n_out * 4, cudaMemcpyDeviceToHost, st));
+    }
+    SVB_CUDA(cudaStreamSynchronize(st));
+    memcpy(wav_host, g->pin_out, n_out * (i16 ? 2 : 4));
+    return SVB_OK;
+}
+}  // namespace
+
+extern "C" int svb_gen_spec2wav_ragged_host(svb_gen_t *g, const float *mel_host, const float *f0_host, const int32_t *lengths_host,
+                                            int32_t B, uint64_t seed, float *wav_host, void *stream) {
+    return spec2wav_ragged(g, "spec2wav_ragged", mel_host, f0_host, lengths_host, B, seed, false, 0, wav_host, stream);
+}
+
+extern "C" int svb_gen_spec2wav_ragged_host_i16(svb_gen_t *g, const float *mel_host, const float *f0_host, const int32_t *lengths_host,
+                                                int32_t B, uint64_t seed, int32_t norm, int16_t *wav_host, void *stream) {
+    return spec2wav_ragged(g, "spec2wav_ragged_i16", mel_host, f0_host, lengths_host, B, seed, true, norm, wav_host, stream);
 }
 
 extern "C" int svb_gen_get_tap(svb_gen_t *g, const char *name, float *out_dev, int64_t capacity_floats, int64_t *shape3,

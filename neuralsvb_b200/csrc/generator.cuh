@@ -142,6 +142,18 @@ struct svb_gen {
     // Lists depend on the stage, the batch / length and the plan's MT; cached per (stage, chain_ordered, MT).
     bool merge = true;              // SVB_MERGE=0: one launch per convolution (round-1 schedule)
     std::map<int, svb::TcWorkList> worklists;
+    std::vector<int> wl_len;        // per-clip lengths the cached lists were built for (empty: uniform batch)
+
+    // ragged batches (svb_gen_forward_ragged): every row >= len[b] * (upsampling so far) of every activation buffer must
+    // read as zero.  hw[b] = frames clip b had in the last forward since the workspace was cleared; a clip that shrinks
+    // gets rows [len, hw) zeroed before the forward.
+    std::vector<int> hw;
+    int *rg_dev = nullptr;          // device table [len B | hw B | off B + 1] of the current ragged forward
+    size_t rg_cap = 0;
+    std::vector<int> cur_len;       // host copy of len (empty: uniform)
+    const int *cur_len_dev = nullptr;
+    double cur_frames = 0;          // sum of the clips' frames (B * T when uniform): FLOP / byte counts use valid rows only
+    int cur_T = 1;
 
     bool profile = false;
     std::vector<LaunchRec> recs;

@@ -51,6 +51,11 @@ struct NsfDims {
     int T;              // F * U samples
     int nchunk;         // ceil(T / 32)
     float sr;
+    // ragged batch (nullptr = every clip F frames): clip b has len[b] frames; with `off`, its f0 starts at f0[off[b]]
+    // (packed, clip after clip) instead of f0[b * F].  Every scan starts at t = 0 of the clip, as in a one-clip call.
+    const int *len, *off;
+    __device__ int frames(int b) const { return len ? len[b] : F; }
+    __device__ const float *f0_of(const float *f0, int b) const { return f0 + (off ? (size_t)off[b] : (size_t)b * F); }
 };
 
 // initial phase: rand_ini[b][k] (k = 0 forced to 0, :54) or Philox uniform
@@ -71,21 +76,22 @@ __global__ void nsf_frame_prefix_kernel(NsfDims d, const float *__restrict__ f0,
     const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (wid >= d.B * kH) return;
     const int b = wid / kH, k = wid % kH;
-    const float *f0b = f0 + (size_t)b * d.F;
+    const float *f0b = d.f0_of(f0, b);
+    const int Fb = d.frames(b);
     double *out = base1 + (size_t)wid * d.F;
     const float rad0 = rad_of(f0b[0], k, d.sr);
     const float r0p = rad0 + rand_ini_of(rand_ini, seed, b, k);   // fp32 add (:56)
     double carry = (double)r0p - (double)rad0;
-    for (int f0i = 0; f0i < d.F; f0i += 32) {
+    for (int f0i = 0; f0i < Fb; f0i += 32) {
         const int f = f0i + lane;
-        double v = (f < d.F) ? (double)d.U * (double)rad_of(f0b[f], k, d.sr) : 0.0;
+        double v = (f < Fb) ? (double)d.U * (double)rad_of(f0b[f], k, d.sr) : 0.0;
         double incl = v;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
             const double n = __shfl_up_sync(0xffffffffu, incl, o);
             if (lane >= o) incl += n;
         }
-        if (f < d.F) out[f] = carry + (incl - v);
+        if (f < Fb) out[f] = carry + (incl - v);
         carry += __shfl_sync(0xffffffffu, incl, 31);
     }
 }
@@ -113,10 +119,15 @@ __global__ void nsf_chunk_sum_kernel(NsfDims d, const float *__restrict__ f0, co
     if (wid >= (long long)d.B * kH * d.nchunk) return;
     const int chunk = (int)(wid % d.nchunk);
     const int bk = (int)(wid / d.nchunk), b = bk / kH, k = bk % kH;
-    const float *f0b = f0 + (size_t)b * d.F;
+    const int Tb = d.frames(b) * d.U;
+    if (chunk * 32 >= Tb) {                                   // past the clip: contributes nothing to its scan
+        if (lane == 0) csum[wid] = 0.0;
+        return;
+    }
+    const float *f0b = d.f0_of(f0, b);
     const float r0p = rad_of(f0b[0], k, d.sr) + rand_ini_of(rand_ini, seed, b, k);
     const int t = chunk * 32 + lane;
-    double v = (t < d.T) ? nsf_v(d, f0b, base1 + (size_t)bk * d.F, k, t, r0p) : 0.0;
+    double v = (t < Tb) ? nsf_v(d, f0b, base1 + (size_t)bk * d.F, k, t, r0p) : 0.0;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     if (lane == 0) csum[wid] = v;
@@ -151,9 +162,11 @@ __global__ void nsf_synth_kernel(NsfDims d, const float *__restrict__ f0, const 
     const int lane = threadIdx.x & 31;
     if (wid >= (long long)d.B * d.nchunk) return;
     const int chunk = (int)(wid % d.nchunk), b = (int)(wid / d.nchunk);
-    const float *f0b = f0 + (size_t)b * d.F;
+    const int Tb = d.frames(b) * d.U;
+    if (chunk * 32 >= Tb) return;                             // past the clip: har there is never read
+    const float *f0b = d.f0_of(f0, b);
     const int t = chunk * 32 + lane;
-    const bool valid = t < d.T;
+    const bool valid = t < Tb;
     const float f0t = valid ? f0b[t / d.U] : 0.f;
     const float uv = f0t > 0.f ? 1.f : 0.f;                                   // _f02uv (:38-42), threshold 0
     const float noise_amp = uv * 0.003f + (1.f - uv) * 0.1f / 3.f;            // (:131)
@@ -202,9 +215,9 @@ size_t nsf_workspace_bytes(int B, int F, int U) {
 
 int launch_nsf_source(const float *f0, const float *rand_ini, const float *noise, uint64_t seed, int B, int F, int U,
                       float sr, const float *lin_w_dev, const float *lin_b_dev, void *workspace, float *har, float *sines,
-                      cudaStream_t st, int *launches) {
+                      cudaStream_t st, int *launches, const int *len, const int *off) {
     NsfDims d;
-    d.B = B, d.F = F, d.U = U, d.T = F * U, d.nchunk = (d.T + 31) / 32, d.sr = sr;
+    d.B = B, d.F = F, d.U = U, d.T = F * U, d.nchunk = (d.T + 31) / 32, d.sr = sr, d.len = len, d.off = off;
     double *base1 = reinterpret_cast<double *>(workspace);
     double *csum = base1 + (size_t)B * kH * F;
     const int tpb = 128;

@@ -174,10 +174,16 @@ class HifiGanGenerator(nn.Module):
         self._drop_handle()
         return r
 
-    def forward(self, x, f0=None, rand_ini=None, noise=None, seed=None):
+    def forward(self, x, f0=None, rand_ini=None, noise=None, seed=None, lengths=None):
         """x [B, n_mel, T] fp32 on a CUDA device, f0 [B, T] Hz or None -> [B, 1, T*hop].
         ``rand_ini`` [B,9] / ``noise`` [B,T*hop,9] inject the NSF source's random draws
         (parity testing); otherwise they are drawn in-kernel from ``seed``.
+
+        ``lengths`` (list, or CPU / CUDA integer tensor [B], 1 <= lengths[b] <= T): a ragged batch in one launch
+        sequence (svb_gen_forward_ragged).  Clip b's first ``lengths[b]*hop`` samples equal a forward of
+        ``x[b:b+1, :, :lengths[b]]`` alone (same injected noise); the rest of its row is 0 and nothing of ``x`` / ``f0`` /
+        ``noise`` past its length is read.  The schedule is built on the host, so a CUDA tensor costs one device-to-host
+        copy (and a sync).  Inference only: with grad in ``train()`` mode it raises ``NotImplementedError``.
 
         In ``train()`` mode with grad enabled the result carries a grad_fn: ``backward`` runs
         ``svb_gen_backward`` (native data / weight gradients) and hands every parameter its gradient
@@ -190,11 +196,13 @@ class HifiGanGenerator(nn.Module):
             self.seed += 1
             seed = self.seed
         if train:
+            if lengths is not None:
+                raise NotImplementedError('ragged batches (lengths=...) are inference only: the training tape takes clips of equal length')
             entries = self._param_entries()
             return _GenTrainFn.apply(self, x, f0, rand_ini, noise, seed, *[p for e in entries for p in e[2]])
-        return self._run_forward(x, f0, rand_ini, noise, seed, train=False)
+        return self._run_forward(x, f0, rand_ini, noise, seed, train=False, lengths=lengths)
 
-    def _run_forward(self, x, f0, rand_ini, noise, seed, train):
+    def _run_forward(self, x, f0, rand_ini, noise, seed, train, lengths=None):
         lib = _native.lib()
         g = self._ensure_handle(x.device)
         g = self._sync_weights(g, train)
@@ -207,10 +215,24 @@ class HifiGanGenerator(nn.Module):
         y = torch.empty(B, 1, T * hop, device=x.device, dtype=torch.float32)
         ri = None if rand_ini is None else rand_ini.contiguous().float().to(x.device)
         nz = None if noise is None else noise.contiguous().float().to(x.device)
+        if lengths is not None:
+            if torch.is_tensor(lengths):
+                lengths = lengths.detach().to('cpu')           # the one device-to-host copy of a CUDA tensor
+            lens = np.ascontiguousarray(np.asarray(lengths).reshape(-1), dtype=np.int64)
+            if lens.shape != (B,):
+                raise ValueError(f'lengths has {lens.size} entries for a batch of {B}')
+            if (lens < 1).any() or (lens > T).any():
+                raise ValueError(f'lengths must lie in [1, {T}], got {lens.tolist()}')
+            lens = lens.astype(np.int32)
         with torch.cuda.device(x.device):
             st = _native.current_stream_ptr(x.device)
-            _native.check(lib.svb_gen_forward(g, _native.ptr(x), _native.ptr(f0), _native.ptr(ri), _native.ptr(nz),
-                                              ctypes.c_uint64(seed), B, T, _native.ptr(y), st), 'gen_forward')
+            if lengths is None:
+                _native.check(lib.svb_gen_forward(g, _native.ptr(x), _native.ptr(f0), _native.ptr(ri), _native.ptr(nz),
+                                                  ctypes.c_uint64(seed), B, T, _native.ptr(y), st), 'gen_forward')
+            else:
+                _native.check(lib.svb_gen_forward_ragged(g, _native.ptr(x), _native.ptr(f0), lens.ctypes.data_as(ctypes.c_void_p),
+                                                         _native.ptr(ri), _native.ptr(nz), ctypes.c_uint64(seed), B, T,
+                                                         _native.ptr(y), st), 'gen_forward_ragged')
         return y
 
     # ------------------------------------------------------------------ training

@@ -150,6 +150,49 @@ class HifiGAN(BaseVocoder):
             out = np.stack([denoise(o, v=hparams['vocoder_denoise_c']) for o in out])
         return out
 
+    def spec2wav_ragged(self, mels, f0s=None, seed=None, int16=False, norm=False):
+        """Clips of different lengths in one call: list of mel [T_b, n_mel] (host arrays), f0s list of [T_b] or None ->
+        list of np.float32 [T_b*hop] (np.int16 with ``int16=True``).  One H2D of the packed clips, one ragged generator
+        forward, one D2H (svb_gen_spec2wav_ragged_host[_i16]); clip b equals ``forward(..., lengths=...)`` on the padded batch.
+        The float path applies ``denoise`` per clip when ``vocoder_denoise_c > 0``; ``norm`` takes each clip's own peak."""
+        mels = [np.ascontiguousarray(m, dtype=np.float32) for m in mels]
+        if not mels:
+            return []
+        lens = np.array([m.shape[0] for m in mels], np.int32)
+        if any(m.ndim != 2 or m.shape[1] != mels[0].shape[1] for m in mels):
+            raise ValueError('every mel must be [T_b, n_mel] with the same n_mel')
+        cat = np.ascontiguousarray(np.concatenate(mels))
+        f0cat = None
+        if f0s is not None:
+            f0s = [np.asarray(f, dtype=np.float32).reshape(-1) for f in f0s]
+            if [len(f) for f in f0s] != lens.tolist():
+                raise ValueError('f0s must have one [T_b] array per mel')
+            f0cat = np.ascontiguousarray(np.concatenate(f0s))
+        lib = _native.lib()
+        g = self.model.native_handle(self.device)
+        hop = int(lib.svb_gen_hop(g))
+        if int16 and hparams.get('vocoder_denoise_c', 0.0) > 0:
+            raise ValueError('int16 output and vocoder_denoise_c > 0 are exclusive (the post-filter works on floats)')
+        out = np.empty(int(lens.sum()) * hop, np.int16 if int16 else np.float32)
+        if seed is None:
+            self.model.seed += 1
+            seed = self.model.seed
+        vp = lambda a: None if a is None else a.ctypes.data_as(ctypes.c_void_p)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            with utils.Timer('hifigan', enable=hparams.get('profile_infer', False)):
+                st = _native.current_stream_ptr(self.device)
+                if int16:
+                    _native.check(lib.svb_gen_spec2wav_ragged_host_i16(g, vp(cat), vp(f0cat), vp(lens), len(mels), ctypes.c_uint64(seed),
+                                                                       int(bool(norm)), vp(out), st), 'spec2wav_ragged_i16')
+                else:
+                    _native.check(lib.svb_gen_spec2wav_ragged_host(g, vp(cat), vp(f0cat), vp(lens), len(mels), ctypes.c_uint64(seed),
+                                                                   vp(out), st), 'spec2wav_ragged')
+        wavs = np.split(out, np.cumsum(lens.astype(np.int64) * hop)[:-1])
+        if not int16 and hparams.get('vocoder_denoise_c', 0.0) > 0:       # vocoders/hifigan.py:66-69, per clip
+            from neuralsvb_b200.vocoders.vocoder_utils import denoise
+            wavs = [denoise(w, v=hparams['vocoder_denoise_c']) for w in wavs]
+        return wavs
+
     @staticmethod
     def wav2spec_batch(wav_fns, hp=None):
         """The binarizer's per-file ``wav2spec`` loop (data_gen/tts/base_binarizer.py:168-178,
